@@ -30,6 +30,9 @@ sys.path.insert(0, ROOT)
 K_GRAPH = 55
 K = K_GRAPH + 1
 READ_LEN = 150
+# --dump-outputs without --buckets: the bucket count decides which bucket every record lands in, so it must not follow the CPU count
+# (10 x host threads) for two runs of the same command to be comparable output for output; 1280 = 10 x 128 threads
+DUMP_BUCKETS = 1280
 
 
 def parse_args():
@@ -39,11 +42,59 @@ def parse_args():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--reads", type=int, default=int(os.environ.get("SGPU_BENCH_READS", 100_000_000)), help="reads per GPU")
-    ap.add_argument("--buckets", type=int, default=0, help="0 = 10 x host threads, as the reference's graph path (construction.cpp:242)")
+    ap.add_argument("--buckets", type=int, default=0, help="0 = 10 x host threads, as the reference's graph path (construction.cpp:242); "
+                                                            "with --dump-outputs, 0 = %d whatever the host" % DUMP_BUCKETS)
     ap.add_argument("--cpu-sample-reads", type=int, default=0, help="reads per reference-arm step; 0 = as many as fit the time budget (calibrated on a 1 M-read run)")
     ap.add_argument("--check-reads", type=int, default=2_000_000, help="N>1: reads per rank of the distributed-vs-single-GPU checksum check (0 = skip)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (bucket sizes, device checksums, a fixed seeded sample "
+                         "of the counted records and of the serialized KMerIndex) as DIR/<name>.npy in float64/float32. The files depend "
+                         "on --reads and --buckets only (and --gpus), not on the host's CPU count")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
+
+
+DUMP_BLOCKS, DUMP_BLOCK = 512, 1024            # records sampled by --dump-outputs: 512 blocks of 1024 consecutive records
+DUMP_INDEX_HEAD, DUMP_INDEX_BLOCKS, DUMP_INDEX_BLOCK = 1 << 16, 256, 4096      # serialized KMerIndex bytes sampled
+
+
+def _halves(a):
+    """u64 values as their (low, high) 32-bit halves in float64, which holds them exactly"""
+    import numpy as np
+    a = np.asarray(a, np.uint64)
+    return np.stack([a & np.uint64(0xFFFFFFFF), a >> np.uint64(32)], axis=-1).astype(np.float64)
+
+
+def dump_outputs(out_dir, st, idx, suffix=""):
+    """what a caller of the timed step receives -- the counted (k+1)-mer set (KMerDiskStorage) and its KMerIndex -- as .npy files of at
+    most ~30 MB in all: the full bucket sizes and the device checksums over every record, and for a fixed seeded sample of record
+    blocks the records, their multiplicities and their MPHF slots; the serialized index as its size and a seeded sample of its bytes"""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(12345)
+    n = st.total_kmers()
+    blk = min(DUMP_BLOCK, n)
+    starts = np.unique((rng.random(DUMP_BLOCKS) * (n - blk + 1)).astype(np.int64)) if n else np.zeros(0, np.int64)
+    keys = np.concatenate([st.kmers(int(s), blk) for s in starts]) if n else np.zeros((0, st.nw), np.uint64)
+    counts = np.concatenate([st.counts(int(s), blk) for s in starts]) if n else np.zeros(0, np.uint32)
+    ser = np.empty(idx.serialized_size(), np.uint8)
+    idx.serialize_into(ser.ctypes.data, ser.size)
+    pos = np.unique((rng.random(DUMP_INDEX_BLOCKS) * max(1, ser.size - DUMP_INDEX_BLOCK)).astype(np.int64))
+    ser_sample = np.concatenate([ser[:DUMP_INDEX_HEAD]] + [ser[p:p + DUMP_INDEX_BLOCK] for p in pos])
+    arrays = {
+        "summary": np.array([n, ser.size, st.num_buckets(), st.k()], np.float64),
+        "bucket_sizes": st.bucket_sizes().astype(np.float64),
+        "kmer_checksums": _halves(st.checksum()),
+        "kmers_sample": _halves(keys).reshape(len(keys), 2 * st.nw),
+        "counts_sample": counts.astype(np.float64),
+        "mphf_slots_sample": idx.seq_idx(keys).astype(np.float64) if len(keys) else np.zeros(0, np.float64),
+        "kmer_index_bytes_sample": ser_sample.astype(np.float32),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
 
 
 def host_threads():
@@ -331,7 +382,7 @@ def main():
     from spades_b200.kmer_index import Context, DeBruijnReadKMerSplitter, KMerDiskCounter, KMerIndexBuilder
 
     T = host_threads()
-    B = args.buckets or 10 * T
+    B = args.buckets or (DUMP_BUCKETS if args.dump_outputs else 10 * T)
     n_reads = args.reads
     genome_len = max(READ_LEN + 1, n_reads)          # 150x coverage like config 3 (100 M reads over 100 Mbp)
     words, offs, lens, nwr = gen_reads_device(torch, n_reads, genome_len, 42 + rank, dev)
@@ -376,19 +427,26 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(stream)
     distinct = instances = passes = 0
-    for _ in range(args.steps):
+    last = None
+    for i in range(args.steps):
         st, idx = step_resident()
         t = ctx.times()
         for kname in phases:
             phases[kname] += t[kname]
         distinct, instances, passes = st.total_kmers(), t["instances"], t["passes"]
-        idx.free(); st.free()
+        if args.dump_outputs and i == args.steps - 1:
+            last = (st, idx)           # read back after the timed region
+        else:
+            idx.free(); st.free()
     e1.record(stream)
     barrier()
     ms = e0.elapsed_time(e1)
     sampler.stop_ev.set(); sampler.join()
     launches = ctx.times()["launches"] - l0
     peak = ctx.times()["peak_bytes"]
+    if last is not None:
+        dump_outputs(args.dump_outputs, *last, suffix="" if world == 1 else "_rank%d" % rank)
+        last[1].free(); last[0].free()
     tms = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(tms, op=dist.ReduceOp.MAX)
@@ -453,7 +511,7 @@ def main():
                 step_storage()
                 torch.cuda.synchronize()
                 e4, e5 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                nst = max(1, min(args.steps, 3))
+                nst = args.steps
                 e4.record(stream)
                 for _ in range(nst):
                     d2h_s = step_storage()

@@ -1,11 +1,12 @@
 """Generates tests/golden/*.npz from the UNMODIFIED reference (oracle/_ref/ref_probe).
 
-Run in the build container only (needs /root/reference to have built oracle/_ref):
+Needs the reference sources to have built oracle/_ref:
     make -C oracle ref && python tests/golden/make_golden.py
-Each fixture holds the input reads and every artefact ref_probe dumps for them, so the oracle and the
-CUDA path can be pinned against reference output on machines without /root/reference.
+Each fixture holds the input reads and every artefact ref_probe dumps for them (key arrays over 1 MB as their SHA-256), so the
+oracle and the CUDA path can be pinned against reference output on machines without the reference.
 """
 import gzip
+import hashlib
 import os
 import subprocess
 import sys
@@ -19,13 +20,13 @@ sys.path.insert(0, ROOT)
 from spades_b200.packing import longest_valid, revcomp, synthetic_reads  # noqa: E402
 
 PROBE = os.path.join(ROOT, "oracle", "_ref", "ref_probe")
-REF = "/root/reference"
 
 
 def ecoli_reads():
+    """the reference's own test data set (src/projects/spades/test_dataset), stored next to this script"""
     reads = []
     for f in ("ecoli_1K_1.fq.gz", "ecoli_1K_2.fq.gz"):
-        lines = gzip.open(os.path.join(REF, "src/projects/spades/test_dataset", f), "rt").read().split("\n")
+        lines = gzip.open(os.path.join(HERE, f), "rt").read().split("\n")
         for i in range(1, len(lines), 4):
             s = longest_valid(lines[i].strip().upper())
             if s:
@@ -105,6 +106,9 @@ def save(name, mode, reads, k, B, early_tc=0, edge_index=None):
         res["ei_chunks"] = np.array([10 * 2])          # run_probe's T = 2: the (k+1)-mer path walks the edges in 10 x T vertex chunks
     if early_tc:
         res["tc_bound"] = np.array([early_tc])
+    for key in ("kpomers", "kmers"):
+        if key in res and res[key].size > (1 << 20):
+            res[key + "_sha256"] = np.frombuffer(hashlib.sha256(res.pop(key).tobytes()).hexdigest().encode(), dtype=np.uint8)
     res["reads"] = np.frombuffer("\n".join(reads).encode(), dtype=np.uint8)
     res["k"] = np.array([k]); res["B"] = np.array([B]); res["mode"] = np.frombuffer(mode.encode(), dtype=np.uint8)
     np.savez_compressed(os.path.join(HERE, name + ".npz"), **res)

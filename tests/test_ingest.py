@@ -1,11 +1,13 @@
 """CPU: the host-side read ingest (spades_b200/csrc/ingest.cpp) -- FASTA/FASTQ(.gz) parsing with kseq semantics, LongestValid,
 2-bit packing, and the reference's binary read-stream format.
-Checked against (1) a line-level Python model on adversarial inputs, (2) the reference's own test data set parsed with Python's
-gzip (build container only), (3) the UNMODIFIED reference reading our .seq/.off through io::BinaryFileSingleStream and writing the
-same reads through SingleReadSeq::BinWrite (oracle/_ref/ref_probe binreads; build container only)."""
+Checked against (1) a line-level Python model on adversarial inputs, (2) the reference's own test data set (ecoli_1K_*.fq.gz, stored
+under tests/golden) parsed with Python's gzip, (3) the UNMODIFIED reference reading our .seq/.off through io::BinaryFileSingleStream
+and writing the same reads through SingleReadSeq::BinWrite, and (4) the reference's parser on seeded awkward files; (3) and (4) as
+oracle/_ref/ref_probe binreads and oracle/_ref/ref_fastx produced them (tests/golden/make_golden_seeded.py)."""
 import gzip
+import hashlib
+import json
 import os
-import subprocess
 
 import numpy as np
 import pytest
@@ -14,9 +16,7 @@ from spades_b200.packing import longest_valid, pack_reads
 from spades_b200.reads_io import read_fastx, read_seqfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-PROBE = os.path.join(ROOT, "oracle", "_ref", "ref_probe")
-REF_FASTX = os.path.join(ROOT, "oracle", "_ref", "ref_fastx")
-ECOLI = "/root/reference/src/projects/spades/test_dataset"
+GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 
 def _model(records):
@@ -109,7 +109,6 @@ def test_truncated_fastq_is_an_error(tmp_path):
         read_fastx(p)
 
 
-@pytest.mark.skipif(not os.path.isdir(ECOLI), reason="reference test data set not present")
 def test_truncated_or_corrupt_gzip_is_an_error_not_a_smaller_read_set(tmp_path):
     """a .gz cut in the middle of the deflate stream (or with flipped bytes) must fail with SGPU_EIO -- zlib's gzread() <= 0 is only a
     clean end of input when gzerror() agrees (ADVICE r01)"""
@@ -133,9 +132,9 @@ def test_truncated_or_corrupt_gzip_is_an_error_not_a_smaller_read_set(tmp_path):
 
 def test_ecoli_test_dataset_matches_python_gzip():
     for f in ("ecoli_1K_1.fq.gz", "ecoli_1K_2.fq.gz"):
-        lines = gzip.open(os.path.join(ECOLI, f), "rt").read().split("\n")
+        lines = gzip.open(os.path.join(GOLDEN, f), "rt").read().split("\n")
         want = _model([[lines[i].strip()] for i in range(1, len(lines), 4)])
-        assert read_fastx(os.path.join(ECOLI, f)).strings() == want
+        assert read_fastx(os.path.join(GOLDEN, f)).strings() == want
 
 
 def test_seqfile_round_trip(tmp_path):
@@ -151,38 +150,33 @@ def test_seqfile_round_trip(tmp_path):
     assert np.array_equal(back.words, b.words) and np.array_equal(back.lens, b.lens)
 
 
-@pytest.mark.skipif(not os.path.exists(PROBE), reason="oracle/_ref/ref_probe not built")
-def test_seqfile_format_against_the_unmodified_reference(tmp_path):
+def seqfile_case_reads():
     rng = np.random.default_rng(3)
-    reads = ["".join(rng.choice(list("ACGT"), int(n))) for n in rng.integers(1, 300, 457)]
-    txt = tmp_path / "reads.txt"
-    open(txt, "w").write("\n".join(reads) + "\n")
+    return ["".join(rng.choice(list("ACGT"), int(n))) for n in rng.integers(1, 300, 457)]
+
+
+def test_seqfile_format_against_the_unmodified_reference(tmp_path):
+    """tests/golden/seqfile_reference.npz: what the reference read from our .seq/.off of these reads (3 portions through the .off
+    index), that .off, and the .seq it wrote for the same reads itself"""
+    reads = seqfile_case_reads()
     fa = tmp_path / "r.fa"
     open(fa, "w").write("".join(">%d\n%s\n" % (i, s) for i, s in enumerate(reads)))
     prefix = str(tmp_path / "lib")
     read_fastx(fa).write_seqfile(prefix)
-    subprocess.check_call([PROBE, "binreads", str(txt), "21", "1", "3", str(tmp_path / "out"), prefix], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-    # the reference reads our files (3 portions through the .off index) ...
-    assert open(prefix + "_readback.txt").read().split() == reads
+    z = np.load(os.path.join(GOLDEN, "seqfile_reference.npz"))
+    # the reference reads our files (the .off index it read is the one we write) ...
+    assert open(prefix + ".off", "rb").read() == z["off"].tobytes()
+    assert z["readback"].tobytes().decode().split() == reads          # guards the fixture: it holds the reads these seeds make
     # ... and writes the same bytes itself, up to the padding bits above the last base of a read: a reference Sequence of <= 60
     # bases lives inline in 16 bytes whose top byte is its metadata (sequence.hpp:194-262), and Sequence::BinWrite dumps that
     # byte along with the data; BinRead restores the metadata afterwards (:808-815), so the padding is "don't care" on input
+    open(prefix + "_ref.seq", "wb").write(z["ref_seq"].tobytes())
     assert _canonical_seqfile(prefix + "_ref.seq") == _canonical_seqfile(prefix + ".seq")
     assert read_seqfile(prefix + "_ref").strings() == reads            # and we read the reference's bytes
 
 
-def _ref_parse(path, tmp_path):
-    out = str(tmp_path / "ref_parsed.txt")
-    subprocess.check_call([REF_FASTX, str(path), out], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-    lines = open(out).read().split("\n")
-    recs = int([l for l in lines if l.startswith("#records")][0].split()[1])
-    return [l for l in lines if l and not l.startswith("#")], recs
-
-
-@pytest.mark.skipif(not os.path.exists(REF_FASTX), reason="oracle/_ref/ref_fastx not built")
-def test_parser_against_the_unmodified_reference_parser(tmp_path):
-    """our ingest against io::FastaFastqGzParser (the reference's vendored kseq + zlib) + io::LongestValid, run live (oracle/_ref/ref_fastx)
-    on well-formed and on deliberately awkward files"""
+def parser_case_files(tmp_path):
+    """well-formed and deliberately awkward FASTA/FASTQ files, and the reference's own test data"""
     rng = np.random.default_rng(7)
     def rnd(n, pn=0.0, lower=0.0):
         s = rng.choice(list("ACGT"), n)
@@ -224,13 +218,18 @@ def test_parser_against_the_unmodified_reference_parser(tmp_path):
             f.write("\n".join(q[j:j + 30] for j in range(0, len(s), 30)) + "\nnoise without markers\n")
     files.append(mq)
     # 5. the reference's own test data
-    if os.path.isdir(ECOLI):
-        files += [os.path.join(ECOLI, "ecoli_1K_1.fq.gz"), os.path.join(ECOLI, "ecoli_1K_2.fq.gz")]
-    for f in files:
-        want, recs = _ref_parse(f, tmp_path)
+    files += [os.path.join(GOLDEN, "ecoli_1K_1.fq.gz"), os.path.join(GOLDEN, "ecoli_1K_2.fq.gz")]
+    return [str(f) for f in files]
+
+
+def test_parser_against_the_unmodified_reference_parser(tmp_path):
+    """our ingest against io::FastaFastqGzParser (the reference's vendored kseq + zlib) + io::LongestValid: the SHA-256 of the reads
+    and the record count oracle/_ref/ref_fastx reported for each file (tests/golden/seeded_reference.json)"""
+    want = json.load(open(os.path.join(GOLDEN, "seeded_reference.json")))["parser"]
+    for f in parser_case_files(tmp_path):
         b = read_fastx(f)
-        assert b.strings() == want, str(f)
-        assert b.records == recs, str(f)
+        w = want[os.path.basename(f)]
+        assert (hashlib.sha256("\n".join(b.strings()).encode()).hexdigest(), b.records) == (w["sha256"], w["records"]), f
 
 
 def test_parser_against_reference_golden(tmp_path):

@@ -1,6 +1,6 @@
 """The reference-side adapters of INTEGRATION.md as real code: integration/gpu_kmer_counter.hpp compiled against the UNMODIFIED
 reference headers into a spades-kmercount-compatible tool (integration/spades_kmercount_gpu.cpp) that links libspades_b200.so.
-The binary is built where /root/reference exists (build container) and travels to the GPU box.
+The binaries are built under oracle/_ref/integration where the reference sources are available, like the rest of oracle/_ref.
 
 CPU: it exists, and without a GPU it refuses loudly (no CPU fallback).
 GPU: reference C++ host code -> C ABI -> CUDA: final_kmers byte-identical to the reference's spades-kmercount golden output, the
@@ -16,9 +16,11 @@ import pytest
 import golden_util as G
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-TOOL = os.path.join(ROOT, "integration", "_build", "spades_kmercount_gpu")
-GBUILDER = os.path.join(ROOT, "integration", "_build", "spades_gbuilder_gpu")
-needs_tool = pytest.mark.skipif(not os.path.exists(TOOL), reason="integration/_build/spades_kmercount_gpu not built (make -C integration; needs /root/reference)")
+BUILT = os.path.join(ROOT, "oracle", "_ref", "integration")
+PROBE = os.path.join(ROOT, "oracle", "_ref", "ref_probe")
+TOOL = os.path.join(BUILT, "spades_kmercount_gpu")
+GBUILDER = os.path.join(BUILT, "spades_gbuilder_gpu")
+needs_tool = pytest.mark.skipif(not os.path.exists(TOOL), reason="oracle/_ref/integration/spades_kmercount_gpu not built (make -C integration; needs the reference sources)")
 
 
 @needs_tool
@@ -34,16 +36,16 @@ def test_tool_refuses_without_gpu():
 
 
 def test_adapter_is_built_where_the_reference_is():
-    if os.path.isdir("/root/reference/src"):
+    if os.path.exists(PROBE):
         assert os.path.exists(TOOL), "run __graft_entry__.build()"
 
 
 def test_construction_phase_subclass_compiles_against_the_reference():
     """integration/construction_gpu_phase.cpp (KMerCountingGpu : Construction::Phase, the pipeline seam) is compiled against the
     UNMODIFIED reference wherever the reference exists; the object must define the phase's run()"""
-    obj = os.path.join(ROOT, "integration", "_build", "construction_gpu_phase.o")
-    if not os.path.isdir("/root/reference/src") and not os.path.exists(obj):
-        pytest.skip("needs /root/reference to build")
+    obj = os.path.join(BUILT, "construction_gpu_phase.o")
+    if not os.path.exists(PROBE) and not os.path.exists(obj):
+        pytest.skip("needs the reference sources to build (oracle/_ref)")
     assert os.path.exists(obj), "run __graft_entry__.build()"
     syms = subprocess.run(["nm", "-C", obj], capture_output=True, text=True).stdout
     assert "KMerCountingGpu::run" in syms and "CoverageFilterGpu::run" in syms and "GpuKMerDiskCounterT<" in syms
@@ -89,7 +91,7 @@ def test_tool_takes_gzipped_fastq_like_the_original():
     assert np.array_equal(fk, g["final_kmers"])
 
 
-@pytest.mark.skipif(not os.path.exists(GBUILDER), reason="integration/_build/spades_gbuilder_gpu not built")
+@pytest.mark.skipif(not os.path.exists(GBUILDER), reason="oracle/_ref/integration/spades_gbuilder_gpu not built")
 def test_gbuilder_tool_refuses_without_gpu():
     import torch
     if torch.cuda.is_available():
@@ -101,7 +103,7 @@ def test_gbuilder_tool_refuses_without_gpu():
     assert p.returncode == 3 and "no CPU fallback" in p.stderr
 
 
-@pytest.mark.skipif(not os.path.exists(GBUILDER), reason="integration/_build/spades_gbuilder_gpu not built")
+@pytest.mark.skipif(not os.path.exists(GBUILDER), reason="oracle/_ref/integration/spades_gbuilder_gpu not built")
 @pytest.mark.gpu
 @pytest.mark.parametrize("name,early_tc", [("ecoli_k21_B40_graph", 0), ("loops_k21_B10_graph", 0), ("ecoli_k55_B16_graph", 0), ("syn_k21_B10_tcgraph", 79)])
 def test_reference_graph_construction_over_gpu_arrays(name, early_tc):

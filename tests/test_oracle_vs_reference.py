@@ -1,88 +1,85 @@
-"""CPU test, build container only: runs the UNMODIFIED reference (oracle/_ref/ref_probe) live on fresh
-seeded inputs and checks the C oracle against every artefact. Skipped where the probe binary is absent."""
+"""CPU test: the C oracle against the UNMODIFIED reference (oracle/_ref/ref_probe) on fresh seeded inputs. The reads are regenerated
+here from their seeds; tests/golden/seeded_reference.json holds what the reference produced for them (the SHA-256 of every artefact,
+the serialized indices with their uninitialised bytes zeroed, and the small integers), written by tests/golden/make_golden_seeded.py."""
+import json
 import os
-import subprocess
-import tempfile
 
 import numpy as np
 import pytest
 
 import golden_util as G
 import oracle as O
-from spades_b200.packing import synthetic_reads
+from spades_b200.packing import pack_reads, revcomp, synthetic_reads
 from test_oracle_golden import oracle_artifacts
 
-PROBE = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "ref_probe")
-pytestmark = pytest.mark.skipif(not os.path.exists(PROBE), reason="oracle/_ref/ref_probe not built (make -C oracle ref)")
+GRAPH = [(21, 16, 11), (31, 5, 12), (55, 30, 13), (63, 9, 14), (77, 4, 15), (127, 6, 16)]
+COUNT = [(21, 16, 21), (55, 16, 22), (100, 3, 23)]
+TIP_CLIPPER = [(21, 16, 3000, 100, 4000, 0.01, 41, 1), (21, 8, 3000, 100, 2000, 0.03, 42, 8), (55, 30, 3000, 150, 5000, 0.01, 43, 3),
+               (77, 4, 1500, 150, 2000, 0.01, 44, 8), (9, 3, 1000, 60, 600, 0.1, 45, 8)]
+COVERAGE_PREFILTER = [(21, 2, 51, 1), (20, 3, 52, 8), (55, 2, 53, 3), (63, 4, 54, 8), (69, 2, 55, 2), (127, 3, 56, 8), (11, 6, 57, 8)]
 
 
-def run_probe(mode, reads, k, B, T=3, early_tc=0):
-    with tempfile.TemporaryDirectory() as d:
-        rf = os.path.join(d, "reads.txt")
-        open(rf, "w").write("\n".join(reads) + "\n")
-        out = os.path.join(d, "out")
-        env = dict(os.environ)
-        if early_tc:
-            env["PROBE_EARLY_TC"] = str(early_tc)
-        subprocess.check_call([PROBE, mode, rf, str(k), str(B), str(T), out], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL, env=env, timeout=600)
-        g = {f.replace(".", "_"): np.frombuffer(open(os.path.join(out, f), "rb").read(), np.uint8)
-             for f in os.listdir(out) if os.path.isfile(os.path.join(out, f))}
-    g.update(k=k, B=B, reads=reads)
-    return g
+def case_id(params):
+    return "_".join(str(p) for p in params)
 
 
-@pytest.mark.parametrize("k,B,seed", [(21, 16, 11), (31, 5, 12), (55, 30, 13), (63, 9, 14), (77, 4, 15), (127, 6, 16)])
+def graph_reads(seed):
+    return synthetic_reads(1500, 150, 3000, 0.01, seed=seed)
+
+
+def count_reads(seed):
+    return synthetic_reads(800, 150, 2000, 0.01, seed=seed)
+
+
+def coverage_prefilter_reads(seed):
+    rng = np.random.default_rng(seed)
+    reads = synthetic_reads(2500, 150, 4000, 0.01, seed=seed) + synthetic_reads(400, 150, 40000, 0.02, seed=seed + 1)
+    x = "".join("ACGT"[i] for i in rng.integers(0, 4, 90))
+    return reads + [x + revcomp(x)] * 3 + ["A" * 150, "AC" * 70, "ACGTACGT"]
+
+
+def count_digests(keys, bsz):
+    return {"final_kmers": G.sha256(np.ascontiguousarray(np.asarray(keys, np.uint64).ravel()).tobytes()),
+            "bucket_sizes": G.sha256(np.asarray(bsz, np.int64).tobytes())}
+
+
+def _want(kind, params):
+    fx = json.load(open(os.path.join(G.GOLDEN_DIR, "seeded_reference.json")))
+    return fx[kind][case_id(params)]
+
+
+@pytest.mark.parametrize("k,B,seed", GRAPH)
 def test_oracle_vs_live_reference_graph(k, B, seed):
-    reads = synthetic_reads(1500, 150, 3000, 0.01, seed=seed)
-    g = run_probe("graph", reads, k, B)
-    art, _ = oracle_artifacts(reads, k, B)
-    assert G.check_graph(g, art) == []
+    art, _ = oracle_artifacts(graph_reads(seed), k, B)
+    assert G.graph_digests(art, B) == _want("graph", (k, B, seed))
 
 
-@pytest.mark.parametrize("k,B,seed", [(21, 16, 21), (55, 16, 22), (100, 3, 23)])
+@pytest.mark.parametrize("k,B,seed", COUNT)
 def test_oracle_vs_live_reference_kmercount(k, B, seed):
-    from spades_b200.packing import pack_reads
-    reads = synthetic_reads(800, 150, 2000, 0.01, seed=seed)
-    g = run_probe("count", reads, k, B)
-    words, offs, lens = pack_reads(reads)
+    words, offs, lens = pack_reads(count_reads(seed))
     ks = O.count(words, offs, lens, k, B, 1)
-    assert G.check_count(g, dict(final_kmers=ks.keys, bsz=ks.bsz)) == []
+    assert count_digests(ks.keys, ks.bsz) == _want("count", (k, B, seed))
 
 
-@pytest.mark.parametrize("k,B,n,L,glen,err,seed,T", [(21, 16, 3000, 100, 4000, 0.01, 41, 1), (21, 8, 3000, 100, 2000, 0.03, 42, 8),
-                                                     (55, 30, 3000, 150, 5000, 0.01, 43, 3), (77, 4, 1500, 150, 2000, 0.01, 44, 8),
-                                                     (9, 3, 1000, 60, 600, 0.1, 45, 8)])
+@pytest.mark.parametrize("k,B,n,L,glen,err,seed,T", TIP_CLIPPER)
 def test_oracle_vs_live_reference_early_tip_clipper(k, B, n, L, glen, err, seed, T):
     """the reference's clipper runs racily on T threads; its result (and the oracle's) must not depend on T"""
     reads = synthetic_reads(n, L, glen, err, seed=seed)
-    g = run_probe("graph", reads, k, B, T=T, early_tc=L - k)
     art, r = oracle_artifacts(reads, k, B, early_tc=L - k)
-    assert G.check_graph(g, art) == []
+    assert G.graph_digests(art, B) == _want("early_tip_clipper", (k, B, n, L, glen, err, seed, T))
     assert r["tc"]["removed"] > 0
 
 
-@pytest.mark.parametrize("k,thr,seed,T", [(21, 2, 51, 1), (20, 3, 52, 8), (55, 2, 53, 3), (63, 4, 54, 8), (69, 2, 55, 2), (127, 3, 56, 8), (11, 6, 57, 8)])
+@pytest.mark.parametrize("k,thr,seed,T", COVERAGE_PREFILTER)
 def test_oracle_vs_live_reference_coverage_prefilter(k, thr, seed, T):
     """SURVEY 8f-3: the CoverageFilter phase of the unmodified reference (HLL bound -> qf::cqf -> median filter, filled by T racing
     threads) against the oracle's restatement: the cardinality bound, the key width, the verdict for every read and the rolling hash
     itself, for k+1 below, at and above 64 (rotation by (k+1) mod 64)"""
-    from spades_b200.packing import pack_reads, revcomp
-    rng = np.random.default_rng(seed)
-    reads = synthetic_reads(2500, 150, 4000, 0.01, seed=seed) + synthetic_reads(400, 150, 40000, 0.02, seed=seed + 1)
-    x = "".join("ACGT"[i] for i in rng.integers(0, 4, 90))
-    reads += [x + revcomp(x)] * 3 + ["A" * 150, "AC" * 70, "ACGTACGT"]
-    with tempfile.TemporaryDirectory() as d:
-        rf = os.path.join(d, "reads.txt")
-        open(rf, "w").write("\n".join(reads) + "\n")
-        env = dict(os.environ); env["PROBE_COV_THR"] = str(thr)
-        subprocess.check_call([PROBE, "covfilter", rf, str(k), "4", str(T), os.path.join(d, "out")], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL,
-                              env=env, timeout=600)
-        card, bits, mask, _ = [int(v) for v in open(os.path.join(d, "out", "covfilter.txt")).read().split()]
-        keep_ref = np.array([int(v) for v in open(os.path.join(d, "out", "keep.txt")).read().split()], dtype=np.uint8)
-        hashes = np.fromfile(os.path.join(d, "out", "hashes.bin"), dtype=np.uint64)
+    reads = coverage_prefilter_reads(seed)
+    want = _want("coverage_prefilter", (k, thr, seed, T))
     words, offs, lens = pack_reads(reads)
     keep, st = O.cov_filter(words, offs, lens, k + 1, thr)
-    assert st[0] == card and st[1] == bits and (1 << bits) - 1 == mask
-    assert np.array_equal(keep, keep_ref)
+    assert st[0] == want["card"] and st[1] == want["key_bits"] and (1 << st[1]) - 1 == want["range_mask"]
+    assert G.sha256(np.asarray(keep, np.uint8).tobytes()) == want["keep"]
     hh = [O.cyclic_hash(words[int(offs[i]):], j, k + 1) for i in range(64) for j in range(max(0, len(reads[i]) - k))]
-    assert np.array_equal(np.array(hh, dtype=np.uint64), hashes)
+    assert G.sha256(np.array(hh, dtype=np.uint64).tobytes()) == want["hashes"]
