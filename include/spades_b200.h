@@ -167,7 +167,9 @@ void sgpu_kset_free(sgpu_kset *s);
 int sgpu_mphf_build(sgpu_ctx *ctx, const sgpu_kset *s, sgpu_mphf **out);
 int64_t sgpu_mphf_serialized_size(const sgpu_mphf *m);
 int sgpu_mphf_serialize(const sgpu_mphf *m, uint8_t *out, int64_t cap);
-int sgpu_mphf_lookup(const sgpu_mphf *m, const uint64_t *keys, int64_t n, uint64_t *out_idx);   /* host keys, stored (minimal) form */
+/* host keys, stored (minimal) form. A key of the set gets its slot; any other key gets what KMerIndex::seq_idx gives: -1 (2^64 - 1),
+ * always so when its bucket holds no key, or the slot of some other key of the set */
+int sgpu_mphf_lookup(const sgpu_mphf *m, const uint64_t *keys, int64_t n, uint64_t *out_idx);
 void sgpu_mphf_free(sgpu_mphf *m);
 
 /* kpomers must come from sgpu_count(k+1, B, SGPU_CANONICAL); kmers/kmer_index from sgpu_kmers_from_kpomers / sgpu_mphf_build.
@@ -224,7 +226,8 @@ int64_t sgpu_edge_index_size(const sgpu_edge_index *e);                         
 int64_t sgpu_edge_index_serialized_size(const sgpu_edge_index *e);
 int sgpu_edge_index_serialize(const sgpu_edge_index *e, uint8_t *out, int64_t cap);   /* KMerIndex::serialize bytes */
 int sgpu_edge_index_values(const sgpu_edge_index *e, uint64_t *edge_ids, uint32_t *offsets, int64_t n);   /* slot order */
-int sgpu_edge_index_lookup(const sgpu_edge_index *e, const uint64_t *keys, int64_t n, uint64_t *out_idx);  /* host keys -> slots */
+/* host keys (stored form) -> slots; a K-mer not in the index gets -1 or the slot of some other K-mer, as in sgpu_mphf_lookup */
+int sgpu_edge_index_lookup(const sgpu_edge_index *e, const uint64_t *keys, int64_t n, uint64_t *out_idx);
 void sgpu_edge_index_free(sgpu_edge_index *e);
 
 /* ---- multi-GPU count (one process per GPU; SURVEY 8e). Replaces hpcspades' shared-filesystem + MPI pattern

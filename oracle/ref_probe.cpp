@@ -13,7 +13,8 @@
 // test/debruijn/test_utils.cpp:128-138).
 //
 // usage: ref_probe <mode: count|graph|bench> <reads.txt> <k> <num_buckets> <nthreads> <outdir>   (env PROBE_EARLY_TC=<bound>: graph mode
-//        also runs EarlyTipClipperProcessor before the unitig extraction)
+//        also runs EarlyTipClipperProcessor before the unitig extraction; PROBE_QUERIES=<file>: graph mode also answers index
+//        lookups, see below)
 //   reads.txt: one ACGT read per line (N-trimming is the ingest layer's job)
 #include "io/reads/vector_reader.hpp"
 #include "io/reads/rc_reader_wrapper.hpp"
@@ -89,6 +90,25 @@ template<class Index>
 static void dump_index(const Index &idx, const std::filesystem::path &p) {
     std::ofstream os(p, std::ios::binary);
     idx.BinWrite(os);   // u32 k, then KMerIndex::serialize (kmer_index.hpp:102-108)
+}
+
+// KMerIndex::seq_idx (kmer_index.hpp:88-93) of raw records read from `qpath` (ceil(K/32) u64 words each, the stored form) under the
+// index an IndexWrapper holds; one u64 per record to `out` (-1 = NOT_FOUND). The wrapper keeps its KMerIndex protected
+// (perfect_hash_map.hpp:32-34), so a derived accessor reaches it through a member pointer.
+using SlimIndex = kmers::IndexWrapper<RtSeq, kmers::slim_kmer_index_traits<RtSeq>>;
+struct SlimIndexPeek : SlimIndex {
+    static const KMerIndexT &of(const SlimIndex &w) { return *(w.*(&SlimIndexPeek::index_ptr_)); }
+};
+static void dump_queries(const SlimIndex &idx, unsigned K, const std::string &qpath, const std::filesystem::path &out) {
+    const size_t nw = RtSeq::GetDataSize(K);
+    std::ifstream is(qpath, std::ios::binary);
+    std::vector<uint64_t> rec(nw);
+    std::ofstream os(out, std::ios::binary);
+    const auto &index = SlimIndexPeek::of(idx);
+    while (is.read((char *)rec.data(), (std::streamsize)(nw * 8))) {
+        const uint64_t v = index.seq_idx(RtSeq(K, rec.data()));
+        os.write((const char *)&v, 8);
+    }
 }
 
 int main(int argc, char **argv) {
@@ -235,6 +255,7 @@ int main(int argc, char **argv) {
         std::ofstream all(outdir / "kpomers", std::ios::binary);
         for (unsigned i = 0; i < B; ++i) {
             sz << kpomers.bucket_size(i) << "\n";
+            if (!kpomers.bucket_size(i)) continue;        // inserting an empty streambuf sets failbit and drops all later buckets
             std::ifstream in(kpomers.bucket_file(i)->file(), std::ios::binary);
             all << in.rdbuf();
         }
@@ -307,6 +328,13 @@ int main(int argc, char **argv) {
         }
         std::ofstream hs(outdir / "histogram.txt");
         for (size_t v : hist) hs << v << "\n";
+    }
+    // PROBE_QUERIES=<file>: seq_idx of every record of <file> under the k-mer index (kmer_queries_idx.bin) and of every record of
+    // <file>.kp1 under the (k+1)-mer index (kpomer_queries_idx.bin). Both indices are the ones KMerIndexBuilder::BuildIndex built in
+    // memory above: a deserialized index marks empty buckets as built (BooPHF.h:537-577) and answers absent keys differently.
+    if (const char *q = getenv("PROBE_QUERIES")) {
+        dump_queries(ext, k, q, outdir / "kmer_queries_idx.bin");
+        dump_queries(coverage_map, k + 1, std::string(q) + ".kp1", outdir / "kpomer_queries_idx.bin");
     }
     // PROBE_EDGE_INDEX=<kk> (0 = k+1): the EdgeIndex refill of the pipeline (modules/graph_construction.hpp:74-82, alignment/edge_index.hpp:
     // Refill -> GraphPositionFillingIndexBuilder, assembly_graph/index/edge_index_builders.hpp:274-307). kk == k+1 takes the (k+1)-mers

@@ -426,6 +426,11 @@ uint64_t orc_mphf_lookup(const mphf_t *m, const uint64_t *key) {
     return i == (uint64_t)-1 ? i : m->starts[b] + i;
 }
 
+/* orc_mphf_lookup of n keys of nw words each (one call instead of n from the test harness) */
+void orc_mphf_lookup_many(const mphf_t *m, const uint64_t *keys, int64_t n, uint64_t *out) {
+    for (int64_t i = 0; i < n; ++i) out[i] = orc_mphf_lookup(m, keys + i * m->nw);
+}
+
 uint64_t orc_mphf_nfinal(const mphf_t *m) { uint64_t t = 0; for (int b = 0; b < m->B; ++b) t += m->seg[b].nfinal; return t; }
 
 /* KMerIndex::serialize (kmer_index.hpp:102-108) -> mphf::save (BooPHF.h:514-535) -> bitVector::save (:316-323).

@@ -48,6 +48,9 @@ __device__ __forceinline__ uint64_t level_pos(const MphfDev &m, const Kmer<NW> &
 template <int NW>
 __device__ __forceinline__ uint64_t mphf_lookup_dev(const MphfDev &m, const Kmer<NW> &k) {
     const uint32_t b = kmer_bucket<NW>(k, m.B);
+    // an empty bucket owns no words (its woff is where the next piece starts) and its mphf was never built: NOT_FOUND
+    // (BooPHF.h:425-426,467). A non-empty piece owns >= 8 words; woff has kLevels * B + 1 entries, so b = B - 1 is covered too.
+    if (m.woff[b + 1] == m.woff[b]) return ~0ull;
     LevelHasher lh(xxh3_128<NW>(k));
     for (int l = 0; l < kLevels - 1; ++l) {
         const uint64_t h = lh.next();

@@ -4,7 +4,7 @@ tests/test_oracle_vs_reference.py and of the reference-format tests of tests/tes
     make -C oracle ref && python tests/golden/make_golden_seeded.py        (needs the reference sources to build oracle/_ref)
 
 Writes tests/golden/seeded_reference.json (SHA-256 of every artefact, the serialized indices with their uninitialised bytes zeroed,
-and the small integers) and tests/golden/seqfile_reference.npz (the reference's read-back text of our .seq/.off, that .off, and its
+the small integers, and for the index lookups the SHA-256 of the queries and of the slots returned with the number of NOT_FOUND) and tests/golden/seqfile_reference.npz (the reference's read-back text of our .seq/.off, that .off, and its
 own .seq of the same reads).
 """
 import json
@@ -48,8 +48,27 @@ def graph_digests(reads, k, B, T=3, early_tc=0):
     return G.graph_digests(G.ref_graph_art(g), B)
 
 
+def lookup_digests(k, B, seed):
+    """seq_idx under the reference's in-memory k-mer and (k+1)-mer index (PROBE_QUERIES) of the query sets built from the keys it
+    stored: the graph run is done twice, first for the keys, then with the queries"""
+    reads = V.lookup_reads(seed)
+    g = run_probe("graph", reads, k, B)
+    nw = (k + 32) // 32                      # k odd: a k-mer and a (k+1)-mer have the same number of words
+    qk = V.lookup_queries(np.frombuffer(g["kmers"].tobytes(), np.uint64).reshape(-1, nw), k, 10 * seed + 1)
+    qkp = V.lookup_queries(np.frombuffer(g["kpomers"].tobytes(), np.uint64).reshape(-1, nw), k + 1, 10 * seed + 2)
+    with tempfile.TemporaryDirectory() as d:
+        q = os.path.join(d, "queries")
+        qk.tofile(q)
+        qkp.tofile(q + ".kp1")
+        g = run_probe("graph", reads, k, B, env_extra={"PROBE_QUERIES": q})
+    return {"kmer": V.lookup_digests(qk, np.frombuffer(g["kmer_queries_idx_bin"].tobytes(), np.uint64)),
+            "kpomer": V.lookup_digests(qkp, np.frombuffer(g["kpomer_queries_idx_bin"].tobytes(), np.uint64))}
+
+
 def main():
-    out = {"graph": {}, "count": {}, "early_tip_clipper": {}, "coverage_prefilter": {}, "parser": {}}
+    out = {"graph": {}, "count": {}, "early_tip_clipper": {}, "coverage_prefilter": {}, "parser": {}, "lookup": {}}
+    for p in V.LOOKUP:
+        out["lookup"][V.case_id(p)] = lookup_digests(*p)
     for p in V.GRAPH:
         k, B, seed = p
         out["graph"][V.case_id(p)] = graph_digests(V.graph_reads(seed), k, B)

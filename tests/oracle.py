@@ -33,6 +33,7 @@ def lib():
         L.orc_mphf_build.restype = vp; L.orc_mphf_build.argtypes = [vp]
         L.orc_mphf_free.restype = None; L.orc_mphf_free.argtypes = [vp]
         L.orc_mphf_lookup.restype = u64; L.orc_mphf_lookup.argtypes = [vp, vp]
+        L.orc_mphf_lookup_many.restype = None; L.orc_mphf_lookup_many.argtypes = [vp, vp, i64, vp]
         L.orc_mphf_nfinal.restype = u64; L.orc_mphf_nfinal.argtypes = [vp]
         L.orc_mphf_serialize.restype = i64; L.orc_mphf_serialize.argtypes = [vp, vp]
         L.orc_masks.restype = None; L.orc_masks.argtypes = [vp, vp, vp, i64]
@@ -108,6 +109,13 @@ class Mphf:
     def lookup(self, key_words):
         w = np.ascontiguousarray(key_words, np.uint64)
         return int(lib().orc_mphf_lookup(self.h, _p(w)))
+
+    def lookup_many(self, keys):
+        """seq_idx of every row of keys [n, nw] (stored form); -1 as 2^64 - 1"""
+        w = np.ascontiguousarray(keys, np.uint64).reshape(-1, self.ks.nw)
+        out = np.zeros(max(len(w), 1), np.uint64)
+        lib().orc_mphf_lookup_many(self.h, _p(w), len(w), _p(out))
+        return out[: len(w)]
 
     def nfinal(self):
         return int(lib().orc_mphf_nfinal(self.h))

@@ -17,6 +17,9 @@ COUNT = [(21, 16, 21), (55, 16, 22), (100, 3, 23)]
 TIP_CLIPPER = [(21, 16, 3000, 100, 4000, 0.01, 41, 1), (21, 8, 3000, 100, 2000, 0.03, 42, 8), (55, 30, 3000, 150, 5000, 0.01, 43, 3),
                (77, 4, 1500, 150, 2000, 0.01, 44, 8), (9, 3, 1000, 60, 600, 0.1, 45, 8)]
 COVERAGE_PREFILTER = [(21, 2, 51, 1), (20, 3, 52, 8), (55, 2, 53, 3), (63, 4, 54, 8), (69, 2, 55, 2), (127, 3, 56, 8), (11, 6, 57, 8)]
+# index lookups: far more buckets than keys in most cases (k = 21, 33, 63, 99, 127: one to four words per record), so that many
+# absent keys fall into empty buckets
+LOOKUP = [(21, 5000, 61), (33, 3000, 62), (63, 8000, 63), (99, 2000, 64), (127, 1500, 65)]
 
 
 def case_id(params):
@@ -36,6 +39,22 @@ def coverage_prefilter_reads(seed):
     reads = synthetic_reads(2500, 150, 4000, 0.01, seed=seed) + synthetic_reads(400, 150, 40000, 0.02, seed=seed + 1)
     x = "".join("ACGT"[i] for i in rng.integers(0, 4, 90))
     return reads + [x + revcomp(x)] * 3 + ["A" * 150, "AC" * 70, "ACGTACGT"]
+
+
+def lookup_reads(seed):
+    return synthetic_reads(40, 150, 400, 0.01, seed=seed)
+
+
+def lookup_queries(keys, K, seed):
+    """the query set of one index of a LOOKUP case (tests/query_sets.py), from the keys that index holds"""
+    from query_sets import query_set
+    return query_set(keys, K, (K + 31) // 32, seed)
+
+
+def lookup_digests(queries, idx):
+    idx = np.asarray(idx, np.uint64)
+    return {"queries": G.sha256(np.ascontiguousarray(queries, np.uint64).tobytes()), "n": int(len(queries)),
+            "idx": G.sha256(idx.tobytes()), "not_found": int((idx == np.uint64((1 << 64) - 1)).sum())}
 
 
 def count_digests(keys, bsz):
@@ -83,3 +102,19 @@ def test_oracle_vs_live_reference_coverage_prefilter(k, thr, seed, T):
     assert G.sha256(np.asarray(keep, np.uint8).tobytes()) == want["keep"]
     hh = [O.cyclic_hash(words[int(offs[i]):], j, k + 1) for i in range(64) for j in range(max(0, len(reads[i]) - k))]
     assert G.sha256(np.array(hh, dtype=np.uint64).tobytes()) == want["hashes"]
+
+
+@pytest.mark.parametrize("k,B,seed", LOOKUP)
+def test_oracle_vs_live_reference_index_lookups(k, B, seed):
+    """KMerIndex::seq_idx of stored keys, their reverse complements, one-base substitutions and random keys, under the k-mer and the
+    (k+1)-mer index KMerIndexBuilder::BuildIndex built in memory, against the oracle's orc_mphf_lookup. An absent key whose bucket
+    holds no key is NOT_FOUND there (the bucket's mphf was never built, BooPHF.h:425-426,467)."""
+    want = _want("lookup", (k, B, seed))
+    words, offs, lens = pack_reads(lookup_reads(seed))
+    kp = O.count(words, offs, lens, k + 1, B, 0)
+    km = O.kmers_from_kpomers(kp, B)
+    for name, ks, K, qseed in (("kmer", km, k, 10 * seed + 1), ("kpomer", kp, k + 1, 10 * seed + 2)):
+        q = lookup_queries(ks.keys, K, qseed)
+        got = lookup_digests(q, O.Mphf(ks).lookup_many(q))
+        assert got == want[name], name
+        assert (ks.bsz == 0).sum() > 0 and got["not_found"] > 0
